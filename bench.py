@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — tracks-refined/s of the multi-view refinement solve on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference] [--dump-outputs DIR]
 
 A step = one complete solve of the workload's match graph (every component,
 LM to termination).  At N=1 the workload is BASELINE.json configs[1]
@@ -27,6 +27,11 @@ solve.cc + cost.cc + graph.cc compiled unmodified (-O2) against the shim headers
 (Ceres' minimizer restated, see oracle/build_ref.py), on all host cores, "Solver time" scope
 (thread pool creation -> Wait(), solve.cc:615-638, measured in microseconds by the pool shim).
 Falls back to the oracle port when that binary was not built.
+
+--dump-outputs DIR writes what the last timed step computed, the arrays lfr_plan_download() hands the
+caller, as DIR/<name>.npy in float64: positions [N, 2] and, per component slot, iterations,
+termination, initial_cost and final_cost (at N>1 with a _rank<r> suffix per rank).  The workload is
+generated from a fixed seed, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -68,6 +73,25 @@ def ncu_traffic(workload):
             return json.load(fh).get("dram_bytes_per_step", {}).get(workload)
     except Exception:
         return None
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, suffix=""):
+    """Writes each array as out_dir/<name><suffix>.npy in float64.  Above DUMP_LIMIT bytes in all, every
+    array keeps a fixed, seeded sample of its rows (ascending), and <name><suffix>_rows.npy says which."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT:
+            # half the limit for the sampled rows, at most as much again for their indices
+            k = int(a.shape[0] * (DUMP_LIMIT // 2) / total)
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], size=k, replace=False))
+            np.save(os.path.join(out_dir, name + suffix + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
 
 
 def build_workload(name, seed=None):
@@ -440,7 +464,11 @@ def run_b200(args):
     step_ms = [a.elapsed_time(b) for a, b in ev]
     ms_per_step = float(np.mean(step_ms))
     ms_per_step_median = float(np.median(step_ms))
-    _, st = plan.download(stream)
+    pos, st = plan.download(stream)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(positions=pos, **{k: st[k] for k in ("iterations", "termination",
+                                                                                  "initial_cost", "final_cost")}),
+                     suffix="_rank%d" % rank if world > 1 else "")
     alg_bytes, one_pass = plan.traffic(stream)
     launches = plan.num_launches()
     # clocks are sampled over warm-up + the device-timed region; the sampler stops before the
@@ -585,7 +613,13 @@ def main():
     ap.add_argument("--workload", default="cfg2")
     ap.add_argument("--debug-flags", type=int, default=0,
                     help="lfr_options.debug_flags for A/B experiments (LFR_DBG_*; 0 = the product path)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs is only for the b200 solve (--impl b200)")
     args.workload = {"fountain": "cfg2", "herzjesu": "cfg3"}.get(args.workload, args.workload)
     if args.impl == "reference":
         return run_reference(args)

@@ -8,6 +8,7 @@ infrastructure only, built into a temporary directory) and comparing with the re
 other route: without a CUDA device it stops with an error (no CPU fallback); on a GPU it is compared
 with the same goldens."""
 import importlib.util
+import json
 import os
 import subprocess
 import sys
@@ -16,7 +17,8 @@ import numpy as np
 import pytest
 
 from lfr_b200 import synth, wire
-from test_ref_solve import BAD_COMMAND_LINES, GOLD, LAUNCHER, oracle_pipeline, ref_exe, untimed
+from reference_runs import recorded
+from test_ref_solve import BAD_COMMAND_LINES, GOLD, LAUNCHER, live, oracle_pipeline, reference_command_line, untimed
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PRODUCT = os.path.join(ROOT, "multi-view-refinement", "build", "solve_native")
@@ -87,17 +89,18 @@ def test_banned_images_part_files_and_empty_input(checker_exe, oracle, tmp_path)
     assert untimed(r.stdout) == ["# graph nodes: 0", "# graph edges: 0", "# points with at least one coordinate > 0.5: 0"]
 
 
-@pytest.mark.parametrize("argv", BAD_COMMAND_LINES + [["--matches_file=a", "--output_file", "b", "--help=1"]])
+COMMAND_LINES = BAD_COMMAND_LINES + [["--matches_file=a", "--output_file", "b", "--help=1"]]
+
+
+@pytest.mark.parametrize("argv", COMMAND_LINES)
 def test_command_line_errors_match_the_python_launcher_and_the_reference(product_exe, argv):
     """Argument handling needs neither a GPU nor the checker: the PRODUCT binary against the Python
-    launcher (itself compared with the reference binary in test_ref_solve.py) and, where it is built,
-    against the reference binary directly."""
+    launcher and against the reference binary's recorded answer."""
     a = run(product_exe, argv)
     b = subprocess.run([sys.executable, LAUNCHER] + argv, capture_output=True, text=True)
     assert (a.returncode, a.stdout, a.stderr) == (b.returncode, b.stdout, b.stderr)
-    if os.path.exists(os.path.join(ROOT, "oracle", "_ref", "solve")) or os.path.isdir("/root/reference"):
-        c = subprocess.run([ref_exe()] + argv, capture_output=True, text=True)
-        assert (a.returncode, a.stdout, a.stderr) == (c.returncode, c.stdout, c.stderr)
+    c = recorded("command_line", json.dumps(argv), live(reference_command_line, argv))
+    assert (a.returncode, a.stdout, a.stderr) == (c["returncode"], c["stdout"], c["stderr"])
 
 
 def test_unparsable_and_unwritable(product_exe, checker_exe, tmp_path):

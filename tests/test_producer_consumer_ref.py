@@ -1,7 +1,10 @@
-"""SURVEY 8f rows 3-4 against the reference's OWN scripts (imported / executed from /root/reference):
+"""SURVEY 8f rows 3-4 against the reference's OWN scripts:
 
   consumer.import_features   vs  reconstruction-scripts/colmap_utils.py::import_features
   producer.MatchGraphWriter  vs  the proto-building block of two-view-refinement/compute_match_graph.py:163-205
+
+What the scripts produced on each test input is recorded in tests/golden/reference_runs.json; where
+the reference sources are present the scripts are also run and checked against that record.
 
 The reference scripts need `types_pb2` (protoc output, not in the reference tree or this image): the
 runtime-built descriptor classes of tests/proto_runtime.py are injected under that module name.  Two
@@ -10,7 +13,6 @@ things the scripts themselves cannot do in this image are patched in the TEST, n
 """
 import importlib.util
 import os
-import shutil
 import sqlite3
 import sys
 import textwrap
@@ -21,10 +23,15 @@ import pytest
 
 from lfr_b200 import consumer, producer, synth, wire
 from lfr_b200.solver import assemble_solution
+from reference_runs import as_json, recorded, sha256
 
 REF = os.environ.get("LFR_REFERENCE_DIR", "/root/reference")
-needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "reconstruction-scripts", "colmap_utils.py")),
-                               reason="reference sources not available here")
+HAVE_REF = os.path.exists(os.path.join(REF, "reconstruction-scripts", "colmap_utils.py"))
+
+
+def live(fn, *args):
+    """fn(*args) deferred for reference_runs.recorded(), or None where the reference scripts are absent."""
+    return (lambda: fn(*args)) if HAVE_REF else None
 
 
 def _types_pb2():
@@ -64,16 +71,18 @@ def _make_database(path, image_names):
 
 
 def _dump(path):
+    """The tables import_features writes, rows sorted, blobs by their sha256."""
     con = sqlite3.connect(path)
-    out = {t: sorted(con.execute("SELECT * FROM %s" % t).fetchall()) for t in ("keypoints", "matches", "descriptors")}
+    out = {t: [[sha256(x) if isinstance(x, bytes) else x for x in row]
+               for row in sorted(con.execute("SELECT * FROM %s" % t).fetchall())]
+           for t in ("keypoints", "matches", "descriptors")}
     con.close()
     return out
 
 
-@needs_ref
-@pytest.mark.parametrize("with_solution", [True, False])
-def test_import_features_equals_the_reference_script(tmp_path, oracle, with_solution):
-    ref = _load_reference_colmap_utils()
+def write_import_features_case(tmp_path, oracle, with_solution):
+    """Feature files, a two-part matches file and (with_solution) a SolutionFile; returns the arguments
+    import_features needs besides the database."""
     ms = synth.generate("cfg2", scale=0.03, seed=17)
     # a duplicated pair exercises "first pair id wins"; an image without any match exercises the no-entry path
     ms = ms.select_pairs(np.concatenate([np.arange(ms.n_pairs), [3]]))
@@ -102,13 +111,27 @@ def test_import_features_equals_the_reference_script(tmp_path, oracle, with_solu
         fact[0] = 1.5
         with open(sfile, "wb") as fh:
             fh.write(wire.encode_solution(sol.image_names, fact, sol.img_ptr, sol.feature_idx, sol.di, sol.dj))
-    db_ref, db_mine = str(tmp_path / "ref.db"), str(tmp_path / "mine.db")
-    _make_database(db_ref, names)
-    shutil.copy(db_ref, db_mine)
-    r = ref.import_features("/nonexistent", "sift", db_ref, str(img_dir), "unused", str(mfile), sfile)
+    return names, img_dir, mfile, sfile
+
+
+def reference_import_features(tmp_path, names, img_dir, mfile, sfile):
+    ref = _load_reference_colmap_utils()
+    db = str(tmp_path / "ref.db")
+    _make_database(db, names)
+    r = ref.import_features("/nonexistent", "sift", db, str(img_dir), "unused", str(mfile), sfile)
+    return {"return": r, "tables": _dump(db)}
+
+
+@pytest.mark.parametrize("with_solution", [True, False])
+def test_import_features_equals_the_reference_script(tmp_path, oracle, with_solution):
+    names, img_dir, mfile, sfile = case = write_import_features_case(tmp_path, oracle, with_solution)
+    ref = recorded("import_features", "with_solution=%s" % with_solution,
+                   live(reference_import_features, tmp_path, *case))
+    db_mine = str(tmp_path / "mine.db")
+    _make_database(db_mine, names)
     m = consumer.import_features("/nonexistent", "sift", db_mine, str(img_dir), "unused", str(mfile), sfile, run_colmap=False)
-    assert r == m
-    a, b = _dump(db_ref), _dump(db_mine)
+    assert ref["return"] == as_json(m)
+    a, b = ref["tables"], _dump(db_mine)
     assert a["keypoints"] == b["keypoints"] and len(a["keypoints"]) == len(names)
     assert a["matches"] == b["matches"] and len(a["matches"]) > 0
     assert a["descriptors"] == b["descriptors"] == []
@@ -135,9 +158,7 @@ def _reference_emit(pairs, output_file, dump_interval):
     ns["run"](pairs, types.SimpleNamespace(output_file=output_file), mf, dump_interval)
 
 
-@needs_ref
-@pytest.mark.parametrize("dump_interval,n_pairs", [(5000, 7), (3, 7), (3, 6), (2, 1)])
-def test_match_graph_writer_equals_the_reference_loop(tmp_path, dump_interval, n_pairs, monkeypatch):
+def writer_pairs(dump_interval, n_pairs):
     rng = np.random.default_rng(dump_interval * 100 + n_pairs)
     pairs = []
     for k in range(n_pairs):
@@ -152,20 +173,33 @@ def test_match_graph_writer_equals_the_reference_loop(tmp_path, dump_interval, n
             g12[1] = 0.0                                             # SKIP_REFINEMENT-style zero grids (:150-152)
         pairs.append(("img%d.png" % (k % 3), float(1 + 0.25 * (k % 3)), "img%d.png" % (k % 3 + 1), 1.0,
                       matches, sim, g12, g21))
-    ref_dir, my_dir = tmp_path / "ref", tmp_path / "mine"
+    return pairs
+
+
+def reference_writer_files(tmp_path, pairs, dump_interval):
+    """The files the reference's loop writes, as {name: hex bytes}."""
+    ref_dir = tmp_path / "ref"
     ref_dir.mkdir()
-    my_dir.mkdir()
     # the reference's loop hard-codes dump_interval = 5000 (:77-78); the harness passes it in
     _reference_emit(pairs, str(ref_dir / "m.pb"), dump_interval)
+    return {f: (ref_dir / f).read_bytes().hex() for f in sorted(os.listdir(ref_dir))}
+
+
+@pytest.mark.parametrize("dump_interval,n_pairs", [(5000, 7), (3, 7), (3, 6), (2, 1)])
+def test_match_graph_writer_equals_the_reference_loop(tmp_path, dump_interval, n_pairs):
+    pairs = writer_pairs(dump_interval, n_pairs)
+    ref = recorded("match_graph_writer", "dump_interval=%d n_pairs=%d" % (dump_interval, n_pairs),
+                   live(reference_writer_files, tmp_path, pairs, dump_interval))
+    my_dir = tmp_path / "mine"
+    my_dir.mkdir()
     w = producer.MatchGraphWriter(str(my_dir / "m.pb"), dump_interval=dump_interval, packed=True)
     for pr in pairs:
         w.add_pair(*pr)
     w.close()
-    ref_files = sorted(os.listdir(ref_dir))
     mine = sorted(f for f in os.listdir(my_dir) if not f.endswith(".npz"))
-    assert ref_files == mine and len(ref_files) >= 1
-    for f in ref_files:
-        assert (ref_dir / f).read_bytes() == (my_dir / f).read_bytes(), f
+    assert sorted(ref) == mine and len(mine) >= 1
+    for f in mine:
+        assert ref[f] == (my_dir / f).read_bytes().hex(), f
     # the packed form holds the same matches as the protobuf parts
     from lfr_b200.matchset import MatchSet
     back = MatchSet.load_npz(str(my_dir / "m.pb.npz"))

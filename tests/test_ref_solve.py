@@ -11,8 +11,13 @@ Ceres' minimizer is the mini-Ceres restatement, the Graclus cut is csrc/lfr_cut.
 build in this image can pin), protobuf / Boost.PO / ThreadPool are functional equivalents.
 
 Rows pinned here (SURVEY 8a): A4, A5, A7, A8, H1-H5 and the drop-in boundary (b).
+
+What the binary produced on each test input is recorded in tests/golden/reference_runs.json, so these
+tests run where it cannot be built; where it can, it is run as well and checked against the record.
 """
+import functools
 import importlib.util
+import json
 import os
 import subprocess
 import sys
@@ -22,20 +27,35 @@ import pytest
 
 from lfr_b200 import build_problem, synth, wire
 from lfr_b200.solver import assemble_solution
+from reference_runs import recorded, sha256
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
 LAUNCHER = os.path.join(ROOT, "multi-view-refinement", "build", "solve")
 
 
-def ref_exe():
+@functools.lru_cache(maxsize=None)
+def find_ref_exe():
+    """oracle/_ref/solve, or None when it is neither built nor buildable here."""
     spec = importlib.util.spec_from_file_location("lfr_build_ref", os.path.join(ROOT, "oracle", "build_ref.py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     try:
         return mod.build_solve()
     except Exception:
+        return None
+
+
+def ref_exe():
+    exe = find_ref_exe()
+    if exe is None:
         pytest.skip("oracle/_ref/solve is not built and the reference sources are not available here")
+    return exe
+
+
+def live(fn, *args):
+    """fn(*args) deferred for reference_runs.recorded(), or None where the reference binary cannot run."""
+    return (lambda: fn(*args)) if find_ref_exe() is not None else None
 
 
 def run_ref(args, env=None):
@@ -59,36 +79,82 @@ def untimed(stdout):
     return [l for l in stdout.splitlines() if " time:" not in l]
 
 
+def reference_run(tmp_path, matches, extra=(), summaries=False):
+    """The reference binary on one MatchingFile: its SolutionFile's sha256, its stdout without the timing
+    lines and, with summaries=True, from the ceres::Solve summaries recorded by the shim: the total of
+    line-search steps and, per problem in the order of its lowest parameter-block address (= lowest
+    node index of the component), the LM iterations and the initial cost without the fixed cost of the
+    all-constant (root-root) blocks, which the C ABI reports without it."""
+    opath, rpath = tmp_path / "ref_solution.pb", tmp_path / "ref_summaries.txt"
+    r = run_ref(["--matches_file", str(matches), "--output_file", str(opath)] + list(extra),
+                env={"LFR_CERES_RECORD_FILE": str(rpath)} if summaries else None)
+    assert r.returncode == 0, r.stderr
+    out = {"solution_sha256": sha256(opath.read_bytes()), "stdout": untimed(r.stdout)}
+    if summaries:
+        # address iterations termination line-search-steps initial-cost final-cost blocks residuals fixed-cost
+        rows = sorted((l.split() for l in rpath.read_text().splitlines()), key=lambda c: int(c[0]))
+        out["iterations"] = [int(c[1]) for c in rows]
+        out["line_search_steps"] = sum(int(c[3]) for c in rows)
+        out["initial_cost"] = [float(c[4]) - float(c[8]) for c in rows]
+    return out
+
+
+def reference_command_line(argv):
+    r = run_ref(argv)
+    return {"returncode": r.returncode, "stdout": r.stdout, "stderr": r.stderr}
+
+
+def scene_key(name, scale, seed):
+    return "%s scale=%g seed=%s" % (name, scale, seed)
+
+
+def write_scene(tmp_path, name, scale, seed):
+    data = wire.encode_matching_file(synth.generate(name, scale=scale, seed=seed))
+    (tmp_path / "m.pb").write_bytes(data)
+    return data, tmp_path / "m.pb"
+
+
+def write_banned_case(tmp_path):
+    """cfg2 at 8 % with two banned images, as one file (m.pb) and as two .part.N files (split.pb)."""
+    ms = synth.generate("cfg2", scale=0.08, seed=21)
+    data = wire.encode_matching_file(ms)
+    (tmp_path / "m.pb").write_bytes(data)
+    # matches split over .part.N files (compute_match_graph.py:189-205, solve.cc:416-424)
+    half = ms.n_pairs // 2
+    for k, part in enumerate([ms.select_pairs(np.arange(0, half)), ms.select_pairs(np.arange(half, ms.n_pairs))]):
+        (tmp_path / ("split.pb.part.%d" % k)).write_bytes(wire.encode_matching_file(part))
+    return data, [ms.image_names[2], ms.image_names[5]]
+
+
+def write_unparsable(tmp_path):
+    bad = tmp_path / "bad.pb"
+    bad.write_bytes(b"\x0a\xff\xff\xff\xff\x0f not a protobuf")
+    return ["--matches_file", str(bad), "--output_file", str(tmp_path / "o.pb")]
+
+
 SCENES = [("cfg1", 1.0, None), ("cfg2", 0.1, 3), ("cfg2", 0.25, 11), ("cfg3", 0.05, 5), ("cfg4", 0.05, 7),
           ("ring60", 0.5, 2)]
 
 
 @pytest.mark.parametrize("name,scale,seed", SCENES)
 def test_solution_file_is_byte_identical_to_the_reference_binary(oracle, tmp_path, name, scale, seed):
-    ms = synth.generate(name, scale=scale, seed=seed)
-    data = wire.encode_matching_file(ms)
-    mpath, opath, rpath = tmp_path / "m.pb", tmp_path / "s.pb", tmp_path / "rec.txt"
-    mpath.write_bytes(data)
-    r = run_ref(["--matches_file", str(mpath), "--output_file", str(opath), "--n_threads", "4"],
-                env={"LFR_CERES_RECORD_FILE": str(rpath)})
-    assert r.returncode == 0, r.stderr
+    data, mpath = write_scene(tmp_path, name, scale, seed)
+    ref = recorded("solve", scene_key(name, scale, seed),
+                   live(reference_run, tmp_path, mpath, ["--n_threads", "4"], True))
     mine, p, st, lines = oracle_pipeline(oracle, data)
-    assert opath.read_bytes() == mine
+    assert sha256(mine) == ref["solution_sha256"]
     # every stdout line except the three timings (solve.cc:484-485,534,549,591,606,670)
-    assert untimed(r.stdout) == [l for l in lines if " time:" not in l]
+    assert ref["stdout"] == [l for l in lines if " time:" not in l]
     # per-problem LM iteration counts: ceres::Solve summaries recorded by the shim, matched to the
     # dispatch slots through the lowest parameter-block address (= lowest node index of the component)
-    rec = np.loadtxt(str(rpath)).reshape(-1, 9)
     sizes = np.diff(p.comp_ptr.astype(np.int64))
     solved = np.nonzero(sizes > 1)[0]
-    assert rec.shape[0] == solved.shape[0]
+    assert len(ref["iterations"]) == solved.shape[0]
     min_node = np.array([p.comp_nodes[p.comp_ptr[c]] for c in solved])       # nodes ascending inside a component
     order_mine = solved[np.argsort(min_node)]
-    order_ref = np.argsort(rec[:, 0])
-    assert np.array_equal(rec[order_ref, 1].astype(np.int64), st["iterations"][order_mine])
-    assert int(rec[:, 3].sum()) == int(st["total_line_search_steps"])
-    # Summary::initial_cost includes the fixed cost of the all-constant (root-root) blocks; the C ABI reports it without
-    np.testing.assert_allclose(rec[order_ref, 4] - rec[order_ref, 8], st["initial_cost"][order_mine], rtol=1e-11, atol=1e-14)
+    assert np.array_equal(np.array(ref["iterations"], np.int64), st["iterations"][order_mine])
+    assert ref["line_search_steps"] == int(st["total_line_search_steps"])
+    np.testing.assert_allclose(ref["initial_cost"], st["initial_cost"][order_mine], rtol=1e-11, atol=1e-14)
 
 
 @pytest.mark.parametrize("name", ["tiny", "linesearch", "fountain_2pct"])
@@ -101,31 +167,14 @@ def test_committed_goldens_are_the_reference_binarys_output(tmp_path, name):
 
 
 def test_banned_images_and_part_files(oracle, tmp_path):
-    ms = synth.generate("cfg2", scale=0.08, seed=21)
-    data = wire.encode_matching_file(ms)
-    banned = [ms.image_names[2], ms.image_names[5]]
-    m = tmp_path / "m.pb"
-    m.write_bytes(data)
-    o = tmp_path / "o.pb"
-    r = run_ref(["--matches_file", str(m), "--output_file", str(o), "--banned_images", banned[0],
-                 "--banned_images=" + banned[1]])
-    assert r.returncode == 0
+    data, banned = write_banned_case(tmp_path)
+    ref = recorded("solve", "banned images", live(reference_run, tmp_path, tmp_path / "m.pb",
+                                                  ["--banned_images", banned[0], "--banned_images=" + banned[1]]))
     mine, _, _, lines = oracle_pipeline(oracle, data, banned=banned)
-    assert o.read_bytes() == mine and untimed(r.stdout) == [l for l in lines if " time:" not in l]
-    # matches split over .part.N files (compute_match_graph.py:189-205, solve.cc:416-424)
-    half = ms.n_pairs // 2
-    parts = [ms.select_pairs(np.arange(0, half)), ms.select_pairs(np.arange(half, ms.n_pairs))] \
-        if hasattr(ms, "select_pairs") else None
-    if parts is None:
-        pytest.skip("MatchSet.select_pairs not available")
-    base = tmp_path / "split.pb"
-    for k, part in enumerate(parts):
-        (tmp_path / ("split.pb.part.%d" % k)).write_bytes(wire.encode_matching_file(part))
-    o2 = tmp_path / "o2.pb"
-    r = run_ref(["--matches_file", str(base), "--output_file", str(o2)])
-    assert r.returncode == 0
+    assert sha256(mine) == ref["solution_sha256"] and ref["stdout"] == [l for l in lines if " time:" not in l]
+    ref2 = recorded("solve", "part files", live(reference_run, tmp_path, tmp_path / "split.pb"))
     mine2, _, _, _ = oracle_pipeline(oracle, data)
-    assert o2.read_bytes() == mine2
+    assert sha256(mine2) == ref2["solution_sha256"]
 
 
 BAD_COMMAND_LINES = [["--help"], ["--matches_file", "x"], ["--foo", "1"], ["pos"], ["--matches_file"],
@@ -138,16 +187,17 @@ BAD_COMMAND_LINES = [["--help"], ["--matches_file", "x"], ["--foo", "1"], ["pos"
 def test_command_line_errors_match_the_reference_binary(argv):
     """solve.cc:379-403 (Boost.Program_options): same exit code, stdout and stderr from the drop-in
     launcher (argument handling needs no GPU)."""
-    a = run_ref(argv)
+    a = recorded("command_line", json.dumps(argv), live(reference_command_line, argv))
     b = subprocess.run([sys.executable, LAUNCHER] + argv, capture_output=True, text=True)
-    assert (a.returncode, a.stdout, a.stderr) == (b.returncode, b.stdout, b.stderr)
+    assert (a["returncode"], a["stdout"], a["stderr"]) == (b.returncode, b.stdout, b.stderr)
 
 
 def test_parse_failure_exit_code(tmp_path):
-    bad = tmp_path / "bad.pb"
-    bad.write_bytes(b"\x0a\xff\xff\xff\xff\x0f not a protobuf")
-    r = run_ref(["--matches_file", str(bad), "--output_file", str(tmp_path / "o.pb")])
-    assert r.returncode == 255 and "Failed to parse proto object." in r.stderr      # return -1, solve.cc:433-436
+    argv = write_unparsable(tmp_path)
+    a = recorded("command_line", "unparsable input", live(reference_command_line, argv))
+    assert a["returncode"] == 255 and "Failed to parse proto object." in a["stderr"]      # return -1, solve.cc:433-436
+    b = subprocess.run([sys.executable, LAUNCHER] + argv, capture_output=True, text=True)
+    assert (a["returncode"], a["stderr"]) == (b.returncode, b.stderr)
 
 
 @pytest.mark.gpu
