@@ -121,14 +121,12 @@ typedef struct lfr_options {
 } lfr_options;
 
 /* lfr_options.debug_flags (b200 only): route components through the fallback tiers, switch the
- * staging / zero-copy mechanisms off, collect per-component cycle counters.  Results do not
- * depend on them (tests/test_gpu_parity.py). */
+ * zero-copy mechanism off, collect per-component cycle counters.  Results do not depend on them
+ * (tests/test_gpu_parity.py).  Other bits are ignored. */
 #define LFR_DBG_FORCE_SMEM_CHOLESKY 0x1 /* every warp-tier component through the shared-memory Cholesky kernel */
 #define LFR_DBG_NO_TILE 0x2             /* no 64/128-thread tile kernels                                       */
-#define LFR_DBG_STAGE_LDG 0x4           /* stage edge records with LDG -> STS instead of TMA bulk copies       */
 #define LFR_DBG_NO_ZERO_COPY 0x8        /* lfr_solve(): copy edges / positions through HBM even when the caller's buffers are pinned */
 #define LFR_DBG_PROFILE 0x10            /* per-component clock64() counters (lfr_debug_plan_cycles)            */
-#define LFR_DBG_TILE_FROM_SHIFT 8       /* bits 8..15 = n: components with more than n unknowns (n <= 32) use the two-warp tile kernel */
 
 /* Optional per-component results, caller-owned, indexed like comp_ptr. Any
  * pointer may be NULL. */

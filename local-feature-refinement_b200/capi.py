@@ -21,8 +21,7 @@ HOST_LIB_PATH = os.path.join(HERE, "csrc", "liblfr_host.so")
 
 LFR_OK = 0
 # lfr_options.debug_flags (include/lfr.h)
-DBG_FORCE_SMEM_CHOLESKY, DBG_NO_TILE, DBG_STAGE_LDG, DBG_NO_ZERO_COPY, DBG_PROFILE = 0x1, 0x2, 0x4, 0x8, 0x10
-DBG_TILE_FROM_SHIFT = 8
+DBG_FORCE_SMEM_CHOLESKY, DBG_NO_TILE, DBG_NO_ZERO_COPY, DBG_PROFILE = 0x1, 0x2, 0x8, 0x10
 TERM_NAMES = {0: "skipped", 1: "gradient_tol", 2: "parameter_tol", 3: "function_tol",
               4: "min_radius", 5: "no_convergence", 6: "failure", 7: "empty"}
 

@@ -29,14 +29,6 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "shared"]
 
 
-def build_variant(out: str, defines) -> str:
-    """Diagnostic variant of the library (e.g. -DLFR_POLY_PROF) next to the product .so."""
-    cmd = [NVCC] + NVCC_FLAGS + ["-D" + d for d in defines] + ["-o", os.path.join(HERE, out)] + \
-          [os.path.join(HERE, s) for s in SOURCES]
-    subprocess.check_call(cmd)
-    return os.path.join(HERE, out)
-
-
 def _stale(out, deps):
     if not os.path.exists(out):
         return True
@@ -84,7 +76,4 @@ def _build_cuda(force: bool = False, verbose: bool = False) -> str:
 
 
 if __name__ == "__main__":
-    if "--poly-prof" in sys.argv:
-        print(build_variant("liblfr_b200_polyprof.so", ["LFR_POLY_PROF"]))
-        sys.exit(0)
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

@@ -4,7 +4,6 @@
 // computes fails with LFR_ENODEV / LFR_ECUDA when no device is usable.
 #include <algorithm>
 #include <chrono>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
@@ -52,9 +51,6 @@ int cuda_code(cudaError_t e) {
   } while (0)
 
 constexpr int kMaxSmemPerBlock = 227 * 1024;
-// Components with more unknowns than this (and <= 32) take the two-warp tile kernel <64, 32> instead of
-// the one-warp register kernel; 32 = never.  Overridden per plan by LFR_TILE_FROM_N.
-constexpr int kTileFromDefault = 32;
 constexpr int kScheduleThreadsMax = 8;  // host threads that classify the dispatch list (build_buckets)
 constexpr int kMaxStreams = 12;
 
@@ -122,14 +118,12 @@ struct DevBuf {
 struct CtaGroup {
   uint32_t first = 0, n = 0, max_free = 0;
   int minb = 2;
-  int smem_vecs = 6;  // how many of the CG arrays (p, w, r, z, y, preconditioner) live in shared memory
 };
 
 struct Bucket {
   uint32_t offset = 0;  // into the bucket-list buffer
   uint32_t n = 0;
   int emax = 0, ncmax = 0, n2max = 0, smem_per_warp = 0, warps = 4;
-  uint64_t scratch_offset = 0;  // tile tier: first double of this launch's global scratch (12 * emax per CTA)
   int variant = 0;  // 0: shared-memory Cholesky kernel (n <= 64); 16 / 32: register Gauss-Jordan kernel (n <= variant)
   bool stages_edges() const { return variant != 0; }  // warp2 / tile tiers pull their edge records into shared memory
 };
@@ -156,7 +150,7 @@ struct lfr_plan {
   uint32_t N = 0, C = 0;
   uint64_t E = 0;
   uint32_t total_slots = 0;
-  DevBuf row_ptr, edges, track, comp, is_root, comp_ptr, comp_nodes, local_of, pos, pos_init, stats, cycles, times, lists, tile_scratch;
+  DevBuf row_ptr, edges, track, comp, is_root, comp_ptr, comp_nodes, local_of, pos, pos_init, stats, cycles, times, lists;
   // `stats` is one block (one memset, one D2H copy): cost0[Cp] cost1[Cp] iter[Cp] term[Cp] ls[Cp] kept[Cp] err[2] pull[2 x u64]
   uint32_t Cp = 0;               // C rounded up to an even count
   bool pos_is_staged = false;    // lfr_solve(): the start point was uploaded straight into `pos`
@@ -245,7 +239,6 @@ struct lfr_plan {
     P.local_of = local_of.as<uint32_t>();
     P.positions = pos.as<double>();
     P.positions_out = zc_positions ? zc_positions : pos.as<double>();
-    P.stage_mode = (opt.debug_flags & LFR_DBG_STAGE_LDG) ? 0 : 1;
     P.pull_ctr = d_pull();
     P.pull_window = 0;  // set by launch_solve for zero-copy staging only
     P.st_iter = d_iter();
@@ -266,7 +259,7 @@ namespace {
 void free_plan(lfr_plan* pl) {
   if (!pl) return;
   DevBuf* bufs[] = {&pl->row_ptr, &pl->edges, &pl->track, &pl->comp, &pl->is_root, &pl->comp_ptr, &pl->comp_nodes,
-                    &pl->local_of, &pl->pos, &pl->pos_init, &pl->stats, &pl->cycles, &pl->times, &pl->lists, &pl->tile_scratch, &pl->L_comps, &pl->L_rec, &pl->L_meta,
+                    &pl->local_of, &pl->pos, &pl->pos_init, &pl->stats, &pl->cycles, &pl->times, &pl->lists, &pl->L_comps, &pl->L_rec, &pl->L_meta,
                     &pl->L_inlist, &pl->L_twin, &pl->L_fdst, &pl->L_bE01, &pl->L_bE23, &pl->L_fdstE, &pl->L_ell_base, &pl->L_scr, &pl->L_q, &pl->L_node, &pl->L_outptr, &pl->L_inptr, &pl->L_freeof,
                     &pl->L_x, &pl->L_xc, &pl->L_lof, &pl->L_vec};
   for (DevBuf* b : bufs) b->release();
@@ -299,18 +292,14 @@ int build_buckets(lfr_plan* pl, const lfr_problem* p) {
   // measured on cfg4: 26 launches instead of 15, same solve time; profiles/r02_tile_tier_occupancy.txt)
   static const int kClass[] = {2048, 3072, 4096, 6144, 8192, 12288, 16384, 24576, 32768, 57344, kMaxSmemPerBlock};
   constexpr int n_class = sizeof(kClass) / sizeof(kClass[0]);
-  // register warp kernel (8..32), register tile kernel (132 = 64 threads x NREG 32; 48, 64: 64 threads;
-  // 80: 128 threads), smem-Cholesky warp kernel (0)
-  static const int kVariant[9] = {8, 16, 24, 32, 132, 48, 64, 80, 0};
-  constexpr int kNV = 9, kV1 = 8, kKeys = kNV * n_class;
+  // register warp kernel (8..32), register tile kernel (48, 64: 64 threads; 80: 128 threads),
+  // smem-Cholesky warp kernel (0)
+  static const int kVariant[8] = {8, 16, 24, 32, 48, 64, 80, 0};
+  constexpr int kNV = 8, kV1 = 7, kKeys = kNV * n_class;
   constexpr uint16_t kNoKey = 0xffff;
-  auto is_tile = [](int vi) { return vi >= 4 && vi <= 7; };
+  auto is_tile = [](int vi) { return vi >= 4 && vi <= 6; };
   const int dbg = pl->opt.debug_flags;
   const bool no_tile = (dbg & LFR_DBG_NO_TILE) != 0;
-  // components with more than tile_from unknowns (and <= 32) go to the two-warp tile kernel
-  // instead of the one-warp kernel (their edge evaluation is split over 64 threads)
-  const int tf = (dbg >> LFR_DBG_TILE_FROM_SHIFT) & 0xff;
-  const int tile_from = no_tile ? 32 : (tf ? tf : kTileFromDefault);
   const bool force_v1 = (dbg & LFR_DBG_FORCE_SMEM_CHOLESKY) != 0;
   const bool force_pcg = pl->opt.linear_solver == 2;
   auto layout_bytes = [&](int vi, int e, int nc, int n2) {
@@ -401,9 +390,8 @@ int build_buckets(lfr_plan* pl, const lfr_problem* p) {
         continue;
       }
       const int e = std::max<int>(1, (int)eup);
-      int vi = (n2 <= 8) ? 0 : (n2 <= 16 ? 1 : (n2 <= 24 ? 2 : (n2 <= 32 ? 3 : (n2 <= 48 ? 5 : (n2 <= 64 ? 6 : (n2 <= 80 ? 7 : kV1))))));
-      if (vi <= 3 && n2 > tile_from && lfr::TileLayout(e, (int)nc, n2).total <= kMaxSmemPerBlock) vi = 4;
-      if (vi >= 5 && is_tile(vi) && (no_tile || lfr::TileLayout(e, (int)nc, n2).total > kMaxSmemPerBlock)) vi = kV1;
+      int vi = (n2 <= 8) ? 0 : (n2 <= 16 ? 1 : (n2 <= 24 ? 2 : (n2 <= 32 ? 3 : (n2 <= 48 ? 4 : (n2 <= 64 ? 5 : (n2 <= 80 ? 6 : kV1))))));
+      if (is_tile(vi) && (no_tile || lfr::TileLayout(e, (int)nc, n2).total > kMaxSmemPerBlock)) vi = kV1;
       if (force_v1) vi = kV1;
       int need = layout_bytes(vi, e, (int)nc, n2);
       if (need > kMaxSmemPerBlock && vi != kV1) {  // the staged records do not fit: the Cholesky warp kernel reads them from global memory
@@ -532,18 +520,7 @@ int prepare_large(lfr_plan* pl, const lfr_problem* p, cudaStream_t s) {
   // size classes by free nodes (upper bound): 104 bytes of CG vectors per free node in shared memory
   // -> 1 / 2 / 4 / 8 components per SM by shared memory; registers cap it at MINB
   static const uint32_t kClassMaxFree[4] = {0xffffffffu, 1008, 504, 250};
-  int minb[4] = {2, 2, 3, 4};
-  if (const char* e = std::getenv("LFR_CTA_MINB")) {  // tuning hook: "2,2,3,4"
-    int a[4];
-    if (std::sscanf(e, "%d,%d,%d,%d", &a[0], &a[1], &a[2], &a[3]) == 4)
-      for (int i = 0; i < 4; ++i) minb[i] = std::min(4, std::max(2, a[i]));
-  }
-  int smem_vecs[4] = {6, 6, 6, 6};
-  if (const char* e = std::getenv("LFR_CTA_SMEM_VECS")) {  // tuning hook: "6,6,6,6"
-    int a[4];
-    if (std::sscanf(e, "%d,%d,%d,%d", &a[0], &a[1], &a[2], &a[3]) == 4)
-      for (int i = 0; i < 4; ++i) smem_vecs[i] = std::min(6, std::max(0, a[i]));
-  }
+  static const int kClassMinb[4] = {2, 2, 3, 4};
   auto class_of = [&](uint32_t nfree) { return nfree > kClassMaxFree[1] ? 0 : (nfree > kClassMaxFree[2] ? 1 : (nfree > kClassMaxFree[3] ? 2 : 3)); };
   pl->cta_groups.clear();
   uint64_t e_off = 0, n_off = 0, f_off = 0, ell_off = 0, s_off = 0;
@@ -551,8 +528,7 @@ int prepare_large(lfr_plan* pl, const lfr_problem* p, cudaStream_t s) {
   for (int cls = 0; cls < 4; ++cls) {
     CtaGroup g;
     g.first = k;
-    g.minb = minb[cls];
-    g.smem_vecs = smem_vecs[cls];
+    g.minb = kClassMinb[cls];
     for (uint32_t i = 0; i < pl->n_large; ++i) {  // dispatch order (largest first) inside a class
       if (class_of(pl->large_free[i]) != cls) continue;
       const uint32_t c = pl->large_slots[i];
@@ -693,15 +669,6 @@ int fill_plan(lfr_plan* pl, const lfr_problem* p, const lfr_options& o, const do
   host_mark(0);
   LFR_TRY(build_buckets(pl, p));  // host work overlaps the copies above
   host_mark(1);
-  {
-    uint64_t scratch = 0;
-    for (Bucket& b : pl->buckets)
-      if (LFR_TILE_SCRATCH_GLOBAL && (b.variant >= 48 || b.variant == 132)) {
-        b.scratch_offset = scratch;
-        scratch += 12ull * (uint64_t)b.emax * b.n;
-      }
-    if (scratch) LFR_TRY(pl->tile_scratch.reserve(sizeof(double) * scratch));
-  }
   // Zero-copy and the CTA tier: its preparation kernel can pull the records it keeps straight from the
   // pinned array, but SM loads over PCIe run at ~15 GB/s against ~50 GB/s for the copy engine
   // (profiles/README.md), so that pays only while those components hold less than ~0.3 of the edges
@@ -759,15 +726,7 @@ int fill_plan(lfr_plan* pl, const lfr_problem* p, const lfr_options& o, const do
 
 // Bytes of zero-copy staging pulls kept outstanding per device (stage_edges): large enough to cover
 // the PCIe bandwidth-delay product, small enough that records arrive in dispatch order.
-// LFR_PULL_WINDOW_KB overrides (0 = unpaced), read once.
-unsigned zero_copy_pull_window() {
-  static const unsigned w = [] {
-    const char* e = std::getenv("LFR_PULL_WINDOW_KB");
-    if (e && *e) return (unsigned)std::strtoul(e, nullptr, 10) * 1024u;
-    return 512u * 1024u;
-  }();
-  return w;
-}
+constexpr unsigned kZeroCopyPullWindow = 512u * 1024u;
 
 int set_kernel_attrs() {
   static bool done_for_device[16] = {};  // per device, guarded by that device's workspace mutex / idempotent otherwise
@@ -791,8 +750,6 @@ int set_kernel_attrs() {
                                 kMaxSmemPerBlock));
   LFR_CUDA(cudaFuncSetAttribute(lfr::solve_warp2_kernel<1, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 kMaxSmemPerBlock));
-  LFR_CUDA(cudaFuncSetAttribute(lfr::solve_tile_kernel<64, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                kMaxSmemPerBlock));
   LFR_CUDA(cudaFuncSetAttribute(lfr::solve_tile_kernel<64, 48>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 kMaxSmemPerBlock));
   LFR_CUDA(cudaFuncSetAttribute(lfr::solve_tile_kernel<64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -813,7 +770,7 @@ int launch_solve(lfr_plan* pl, cudaStream_t s) {
   lfr::DevProblem P_stage = P_hbm;          // edges pulled once into shared memory, possibly from the caller's pinned buffer
   if (pl->zc_edges) {
     P_stage.edges = pl->zc_edges;
-    P_stage.pull_window = zero_copy_pull_window();
+    P_stage.pull_window = kZeroCopyPullWindow;
   }
   const bool hbm_edges_on_copy_stream = pl->zc_edges && pl->edges_in_hbm;
   const int nb = (int)pl->buckets.size();
@@ -830,10 +787,10 @@ int launch_solve(lfr_plan* pl, cudaStream_t s) {
         LFR_CUDA(cudaStreamWaitEvent(bs, pl->ev_fork, 0));
       }
       if (pl->zc_edges && pl->cta_from_hbm) LFR_CUDA(cudaStreamWaitEvent(bs, pl->ev_edges, 0));
-      // dynamic shared memory for the CG vectors of the group's largest component: the first
-      // `smem_vecs` of p, w, r, z, y (2 doubles per free node each) and the preconditioner (3)
-      const size_t per_node = (size_t)std::min(g.smem_vecs, 5) * 2 + (g.smem_vecs >= 6 ? 3 : 0);
-      const size_t cg_bytes = std::min<size_t>(200 * 1024, (size_t)g.max_free * per_node * sizeof(double));
+      // dynamic shared memory for the CG vectors of the group's largest component: p, w, r, z, y
+      // (2 doubles per free node each) and the preconditioner (3); solve_cta_kernel keeps in HBM
+      // whatever does not fit under the 200 KB cap
+      const size_t cg_bytes = std::min<size_t>(200 * 1024, (size_t)g.max_free * 13 * sizeof(double));
       const lfr::CtaComp* comps = pl->L_comps.as<lfr::CtaComp>() + g.first;
       const unsigned smem_doubles = (unsigned)(cg_bytes / sizeof(double));
       // (512-thread CTAs were measured too — profiles/r02_cta_tier_tuning.txt: slower at every size class)
@@ -861,14 +818,11 @@ int launch_solve(lfr_plan* pl, cudaStream_t s) {
     wb.ncmax = b.ncmax;
     wb.n2max = b.n2max;
     wb.smem_per_warp = b.smem_per_warp;
-    wb.scratch = (LFR_TILE_SCRATCH_GLOBAL && (b.variant >= 48 || b.variant == 132)) ? pl->tile_scratch.as<double>() + b.scratch_offset : nullptr;
     const size_t smem = (size_t)b.smem_per_warp * b.warps;
     const unsigned grid = (b.n + b.warps - 1) / b.warps;
     const lfr::DevProblem& P = b.stages_edges() ? P_stage : P_hbm;
     if (!b.stages_edges() && hbm_edges_on_copy_stream) LFR_CUDA(cudaStreamWaitEvent(bs, pl->ev_edges, 0));
-    if (b.variant == 132)
-      lfr::solve_tile_kernel<64, 32><<<b.n, 64, smem, bs>>>(P, pl->K, wb);
-    else if (b.variant == 48)
+    if (b.variant == 48)
       lfr::solve_tile_kernel<64, 48><<<b.n, 64, smem, bs>>>(P, pl->K, wb);
     else if (b.variant == 64)
       lfr::solve_tile_kernel<64, 64><<<b.n, 64, smem, bs>>>(P, pl->K, wb);
@@ -1125,9 +1079,9 @@ int lfr_plan_traffic(lfr_plan* pl, void* stream, uint64_t* algorithmic_bytes, ui
   return LFR_OK;
 }
 
-/* debug (LFR_PROFILE=1): per-slot cycle counters, 8 x uint64 each */
+/* debug (LFR_DBG_PROFILE): per-slot cycle counters, 8 x uint64 each */
 int lfr_debug_plan_cycles(lfr_plan* pl, unsigned long long* out) {
-  if (!pl || !pl->profile) return fail(LFR_EINVAL, "plan was not created with LFR_PROFILE=1");
+  if (!pl || !pl->profile) return fail(LFR_EINVAL, "plan was not created with LFR_DBG_PROFILE");
   LFR_CUDA(cudaSetDevice(pl->device));
   LFR_CUDA(cudaMemcpy(out, pl->cycles.p, sizeof(unsigned long long) * 8 * (size_t)pl->C, cudaMemcpyDeviceToHost));
   return LFR_OK;
@@ -1168,30 +1122,6 @@ int lfr_debug_time_schedule(const lfr_problem* p, const lfr_options* opt, int re
     LFR_TRY(build_buckets(&pl, p));
     best = std::min(best, std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t0).count());
   }
-  if (std::getenv("LFR_SCHED_SPLIT")) {  // diagnostic: the node loop alone
-    double b2 = 1e300;
-    uint64_t sink = 0;
-    for (int r = 0; r < std::max(reps, 1); ++r) {
-      const auto t0 = std::chrono::steady_clock::now();
-      for (uint32_t c = 0; c < p->n_components; ++c) {
-        uint64_t eup = 0; uint32_t nfree = 0;
-        for (uint32_t i = p->comp_ptr[c]; i < p->comp_ptr[c + 1]; ++i) {
-          const uint32_t v = p->comp_nodes[i];
-          eup += p->row_ptr[v + 1] - p->row_ptr[v];
-          nfree += p->is_root[v] ? 0 : 1;
-        }
-        sink += eup * 3 + nfree;
-      }
-      b2 = std::min(b2, std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t0).count());
-    }
-    std::fprintf(stderr, "node loop alone %.1f us (sink %llu)\n", b2, (unsigned long long)sink);
-  }
-  if (std::getenv("LFR_SCHED_DUMP")) {
-    for (const Bucket& b : pl.buckets)
-      std::fprintf(stderr, "bucket variant %3d  n %6u  emax %5d ncmax %4d n2max %3d  smem/warp %6d  warps %d  -> CTAs/SM by smem %d\n", b.variant,
-                   b.n, b.emax, b.ncmax, b.n2max, b.smem_per_warp, b.warps, (int)(kMaxSmemPerBlock / (b.smem_per_warp * b.warps + 1024)));
-    std::fprintf(stderr, "CTA tier: %zu components\n", pl.large_slots.size());
-  }
   if (digest) {  // FNV-1a over everything the launches depend on: the schedule must not depend on the thread count
     uint64_t h = 1469598103934665603ull;
     auto mix = [&](uint64_t v) {
@@ -1220,18 +1150,6 @@ int lfr_debug_last_host_marks(double* out6) {
   for (int i = 0; i < 6; ++i) out6[i] = g_host_marks[i];
   return LFR_OK;
 }
-
-#ifdef LFR_POLY_PROF
-/* diagnostic build only: cycle split of the line-search polynomial (lfr_math.cuh) */
-int lfr_debug_poly_prof(unsigned long long* out16, int reset) {
-  LFR_CUDA(cudaMemcpyFromSymbol(out16, lfr::g_poly_prof, sizeof(unsigned long long) * 16));
-  if (reset) {
-    unsigned long long z[16] = {0};
-    LFR_CUDA(cudaMemcpyToSymbol(lfr::g_poly_prof, z, sizeof(z)));
-  }
-  return LFR_OK;
-}
-#endif
 
 void lfr_plan_destroy(lfr_plan* pl) {
   if (!pl) return;

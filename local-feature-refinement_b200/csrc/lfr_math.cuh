@@ -273,21 +273,6 @@ __device__ __noinline__ int real_roots_in(const double* c, int n, double lo, dou
   return segment_roots(p, 5, crit[0], crit[1], crit[2], ncrit, lo, hi, out, lane);
 }
 
-#ifdef LFR_POLY_PROF
-// Diagnostic build only (-DLFR_POLY_PROF): cycle split of hermite_minimizer, read
-// back with lfr_debug_poly_prof().  [0] coefficients [1] first evaluations
-// [2] grid classification (or quadratic) [3] extremum cells (or cubic level)
-// [4] root solves (or quartic level) [5] final evaluations
-// [6] quintic calls [7] cubic calls [8] Newton iterations [9] bracket_root calls
-// [10] whole cubic-interpolant call
-__device__ unsigned long long g_poly_prof[16];
-#define LFR_PP_TICK(k) do { const long long n__ = clock64(); if (lane == 0) atomicAdd(&g_poly_prof[k], (unsigned long long)(n__ - pp_t)); pp_t = n__; } while (0)
-#define LFR_PP_COUNT(k) atomicAdd(&g_poly_prof[k], 1ull)
-#else
-#define LFR_PP_TICK(k) do {} while (0)
-#define LFR_PP_COUNT(k) do {} while (0)
-#endif
-
 // ---- fixed-degree variants ----------------------------------------------------
 // The same operations in the same order as the generic routines above, with the
 // sizes known at compile time so that every coefficient and root stays in a
@@ -321,9 +306,7 @@ __device__ __forceinline__ double bracket_root_n(const double (&q)[N], double a,
   double xl = fa < 0.0 ? a : b, xh = fa < 0.0 ? b : a;
   double x = a - fa * newton_quotient(b - a, fb - fa);
   if (!(x > fmin(a, b) && x < fmax(a, b))) x = 0.5 * (a + b);
-  LFR_PP_COUNT(9);
   for (int it = 0; it < 100; ++it) {
-    LFR_PP_COUNT(8);
     double f, df;
     horner2_n<N>(q, x, &f, &df);
     if (f == 0.0) return x;
@@ -400,17 +383,13 @@ __device__ __forceinline__ int quadratic_roots_in(double a, double b, double cc,
 }
 
 // Real roots in [lo, hi] of the quartic q (q[0] != 0), ascending
-__device__ __forceinline__ int quartic_roots_in(const double (&q)[5], double lo, double hi, double (&out)[4], int lane,
-                                                long long& pp_t) {
+__device__ __forceinline__ int quartic_roots_in(const double (&q)[5], double lo, double hi, double (&out)[4], int lane) {
   const double d3[4] = {4.0 * q[0], 3.0 * q[1], 2.0 * q[2], q[3]};
   double c0 = 0.0, c1 = 0.0;
   const int n2 = quadratic_roots_in(3.0 * d3[0], 2.0 * d3[1], d3[2], lo, hi, &c0, &c1);
-  LFR_PP_TICK(2);
   double crit[3] = {0.0, 0.0, 0.0};
   const int n3 = segment_roots_n<4, 3>(d3, c0, c1, 0.0, n2, lo, hi, crit, lane);
-  LFR_PP_TICK(3);
   const int n4 = segment_roots_n<5, 4>(q, crit[0], crit[1], crit[2], n3, lo, hi, out, lane);
-  LFR_PP_TICK(4);
   return n4;
 }
 
@@ -435,7 +414,7 @@ __device__ __forceinline__ int quartic_roots_in(const double (&q)[5], double lo,
 // Every root is polished by the same safeguarded Newton as before, from a bracket
 // 31x tighter, so both routes return the same roots up to the last bits.
 __device__ __forceinline__ int quartic_roots_grid(const double (&q)[5], double lo, double hi, double (&out)[4],
-                                                  int lane, long long& pp_t) {
+                                                  int lane) {
   const double w = (hi - lo) * (1.0 / 31.0);
   const double t = lane == 31 ? hi : fma(w, (double)lane, lo);
   double a1 = q[1], a2 = q[2], a3 = q[3], a4 = q[4];
@@ -459,8 +438,7 @@ __device__ __forceinline__ int quartic_roots_grid(const double (&q)[5], double l
     else if (D == 2) kind = Dp == 0 ? 0 : (Dp == 1 ? 2 : 3);
     else if (D == 3) kind = Dp == 0 ? 1 : 3;
   }
-  if (__any_sync(0xffffffffu, bad || kind == 3)) return quartic_roots_in(q, lo, hi, out, lane, pp_t);
-  LFR_PP_TICK(2);
+  if (__any_sync(0xffffffffu, bad || kind == 3)) return quartic_roots_in(q, lo, hi, out, lane);
   // cells with one extremum of q: find it, look at the sign of q there
   int nl = kind == 1 ? 1 : 0;
   double xb = tn, fb = qn, e = 0.0, qe = 0.0;
@@ -476,7 +454,6 @@ __device__ __forceinline__ int quartic_roots_grid(const double (&q)[5], double l
       }
     }
   }
-  LFR_PP_TICK(3);
   double ra = 0.0, rb = 0.0;
   if (nl >= 1) ra = bracket_root_n<5>(q, t, xb, a4, fb);
   if (__any_sync(0xffffffffu, nl == 2)) {
@@ -503,7 +480,6 @@ __device__ __forceinline__ int quartic_roots_grid(const double (&q)[5], double l
       }
     }
   }
-  LFR_PP_TICK(4);
   return cnt;
 }
 
@@ -512,11 +488,6 @@ __device__ __forceinline__ int quartic_roots_grid(const double (&q)[5], double l
 __device__ __noinline__ double hermite_minimizer(double f0, double g0, double x1, double f1, double g1,
                                                  bool three, double x2, double f2, double g2, double lo,
                                                  double hi, int lane) {
-  long long pp_t = 0;
-#ifdef LFR_POLY_PROF
-  pp_t = clock64();
-  if (lane == 0) LFR_PP_COUNT(three ? 6 : 7);
-#endif
   const double h = three ? fmax(x1, x2) : x1;
   const double ih = 1.0 / h;  // the only division by h: t = x * ih
   const double g0h = g0 * h;
@@ -557,7 +528,6 @@ __device__ __noinline__ double hermite_minimizer(double f0, double g0, double x1
   if (three && c[0] != 0.0) {
     // quintic with a full-degree derivative: everything in registers
     const double c6[6] = {c[0], c[1], c[2], c[3], c[4], c[5]};
-    LFR_PP_TICK(0);
     double ox = (lo + hi) / 2.0;
     double ov = poly_eval_n<6>(c6, ox * ih);
     double v = poly_eval_n<6>(c6, tlo);
@@ -566,12 +536,7 @@ __device__ __noinline__ double hermite_minimizer(double f0, double g0, double x1
     if (v < ov) { ov = v; ox = hi; }
     const double der4[5] = {5.0 * c6[0], 4.0 * c6[1], 3.0 * c6[2], 2.0 * c6[3], c6[4]};
     double roots[4] = {0.0, 0.0, 0.0, 0.0};
-    LFR_PP_TICK(1);
-#ifdef LFR_NO_GRID_ROOTS
-    const int nr = quartic_roots_in(der4, tlo, thi, roots, lane, pp_t);
-#else
-    const int nr = quartic_roots_grid(der4, tlo, thi, roots, lane, pp_t);
-#endif
+    const int nr = quartic_roots_grid(der4, tlo, thi, roots, lane);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       if (i < nr && roots[i] >= tlo && roots[i] <= thi) {
@@ -586,7 +551,6 @@ __device__ __noinline__ double hermite_minimizer(double f0, double g0, double x1
         if (v < ov) { ov = v; ox = sx[i]; }
       }
     }
-    LFR_PP_TICK(5);
     return ox;
   }
   if (!three && c[0] != 0.0) {
@@ -615,7 +579,6 @@ __device__ __noinline__ double hermite_minimizer(double f0, double g0, double x1
         if (v < ov) { ov = v; ox = sx[i]; }
       }
     }
-    LFR_PP_TICK(10);
     return ox;
   }
   // MinimizePolynomial: middle, ends, real parts of the roots of p'

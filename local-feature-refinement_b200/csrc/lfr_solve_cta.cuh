@@ -346,10 +346,10 @@ __device__ __forceinline__ double cta_matvec_bcsr(const CtaCtx& C, const double*
 }
 
 // Block-Jacobi PCG for (S H S + D^2) y = S g; dl = -S y.  Returns validity and
-// {model_cost_change, g . dl, |dl|_inf}.
+// {model_cost_change, g . dl, |dl|_inf}.  tph (LFR_DBG_PROFILE only, else nullptr) accumulates the
+// cycles of the four phases of a CG iteration.
 __device__ __forceinline__ bool cta_lm_step(const CtaCtx& C, double radius, const DevConsts& K, double* model_change,
-                                            double* gd, double* dmax, unsigned* cg_iters, bool diag_mode,
-                                            double* worst_res, unsigned* n_maxit, long long* tph = nullptr) {
+                                            double* gd, double* dmax, unsigned* cg_iters, long long* tph) {
   // damping, preconditioner, initial residual
   double bb = 0.0, rz = 0.0, bad = 0.0;
   for (int f = C.tid; f < C.nf; f += C.nt) {
@@ -469,17 +469,6 @@ __device__ __forceinline__ bool cta_lm_step(const CtaCtx& C, double radius, cons
     ++restarts;
   }
   *cg_iters += (unsigned)it;
-  if (diag_mode && ok && bb > 0.0) {  // LFR_PROFILE: true residual |b - A y| / |b| of the returned solution
-    if (it >= max_it) ++*n_maxit;
-    if (C.regular) cta_matvec_bcsr(C, C.y, C.w, C.pblk); else cta_matvec(C, C.y, C.w);
-    double e2 = 0.0, z1 = 0.0, z2 = 0.0;
-    for (int i = C.tid; i < C.n; i += C.nt) {
-      const double d = C.S[i] * C.g[i] - C.w[i];
-      e2 += d * d;
-    }
-    block_sum3(C, e2, z1, z2);
-    *worst_res = fmax(*worst_res, sqrt(e2 / bb));
-  }
   double mc = 0.0, dot = 0.0, nonfinite = 0.0, mx = 0.0;
   for (int i = C.tid; i < C.n; i += C.nt) {
     const double y = C.y[i], si = C.S[i], gi = C.g[i];
@@ -627,8 +616,7 @@ solve_cta_kernel(const DevProblem P, const DevConsts K, const CtaArrays A, const
   const double cost0 = cost;
   double radius = K.radius0, nu = 2.0;
   int iter = 0, n_invalid = 0, term = LFR_TERM_NO_CONVERGENCE;
-  unsigned ls_steps = 0, cg_iters = 0, n_maxit = 0;
-  double worst_res = 0.0;
+  unsigned ls_steps = 0, cg_iters = 0;
   bool success = true;
   auto norms = [&](double* xn2, double* dn2) {
     double a = 0.0, b = 0.0, z = 0.0;
@@ -661,8 +649,7 @@ solve_cta_kernel(const DevProblem P, const DevConsts K, const CtaArrays A, const
     success = false;
     double model_change = 0.0, gd = 0.0, dmax = 0.0;
     if (prof) t_mark = clock64();
-    bool valid = cta_lm_step(C, radius, K, &model_change, &gd, &dmax, &cg_iters, false, &worst_res, &n_maxit,
-                             prof ? tph : nullptr);
+    bool valid = cta_lm_step(C, radius, K, &model_change, &gd, &dmax, &cg_iters, prof ? tph : nullptr);
     if (prof) t_lm += clock64() - t_mark;
     valid = valid && (model_change > 0.0);
     if (!valid) {

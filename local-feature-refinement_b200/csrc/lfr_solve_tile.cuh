@@ -11,13 +11,6 @@
 
 namespace lfr {
 
-// 1: the per-edge evaluation / assembly scratch (96 of 186 bytes per candidate edge) lives in a per-CTA
-// global area instead of shared memory.  Measured on cfg4 (profiles/r02_tile_tier_occupancy.txt): 1.4x
-// the resident components, each 1.3x slower (scratch latency) -> same solve time; left off.
-#ifndef LFR_TILE_SCRATCH_GLOBAL
-#define LFR_TILE_SCRATCH_GLOBAL 0
-#endif
-
 struct TileLayout {
   int stage, bar;
   int x, xc, g, S, dl, H, scr, tup, prow, red, hdr;
@@ -35,16 +28,11 @@ struct TileLayout {
     S = o; o += 8 * n2max;
     dl = o; o += 8 * n2max;
     H = o; o += 8 * n2max * ldh;
-    // scr (7 doubles per candidate edge: the staged evaluation) and tup (5: the assembly tuples) live
-    // in a per-CTA global scratch area (WarpBucket::scratch), not here: at 96 of 186 bytes per edge they
-    // were what held this tier to 1-2 CTAs (2-4 warps) per SM on ETH3D-scale scenes
-#if LFR_TILE_SCRATCH_GLOBAL
-    scr = 0;
-    tup = 0;
-#else
+    // scr (7 doubles per candidate edge: the staged evaluation) and tup (5: the assembly tuples), 96 of
+    // 186 bytes per edge.  Moving them to a per-CTA global area was measured on cfg4
+    // (profiles/r02_tile_tier_occupancy.txt): 1.4x the resident components, each 1.3x slower -> same time.
     scr = o; o += 8 * 7 * emax;
     tup = o; o += 8 * 5 * emax;
-#endif
     o = align_up(o, 16);
     prow = o; o += 8 * 4 * 84;   // double-buffered pair of pivot rows: 2 x 2 x (80 columns, rhs, spare)
     red = o; o += 8 * 3 * 4;     // block reductions (<= 4 warps)
@@ -387,13 +375,8 @@ solve_tile_kernel(const DevProblem P, const DevConsts K, const WarpBucket B) {
   C.S = (double*)(base + L.S);
   C.dl = (double*)(base + L.dl);
   C.H = (double*)(base + L.H);
-#if LFR_TILE_SCRATCH_GLOBAL
-  C.scr = B.scratch + (size_t)blockIdx.x * 12 * (size_t)B.emax;  // global (L1/L2-resident): lanes <-> edges, SoA
-  C.tup = C.scr + 7 * (size_t)B.emax;
-#else
   C.scr = (double*)(base + L.scr);
   C.tup = (double*)(base + L.tup);
-#endif
   C.prow = (double*)(base + L.prow);
   C.red = (double*)(base + L.red);
   int* hdr = (int*)(base + L.hdr);

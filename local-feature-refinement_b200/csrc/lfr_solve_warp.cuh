@@ -37,8 +37,6 @@ struct DevProblem {
                              // (zero-copy write-back: only free nodes are written, solve.cc:131-141)
   unsigned long long* pull_ctr;  // [2] bytes of staging pulls {ticketed, arrived} (zero-copy pacing, see stage_edges)
   unsigned pull_window;      // 0 = unpaced; else at most this many bytes of staging pulls are outstanding per device
-  int stage_mode;            // how the staging tiers pull a component's edge records into shared memory:
-                             // 1 = TMA 1-D bulk copies (cp.async.bulk + mbarrier), 0 = LDG -> STS
   // per dispatch slot
   int32_t* st_iter;
   int32_t* st_term;
@@ -57,7 +55,6 @@ struct WarpBucket {
   int ncmax;   // max nodes
   int n2max;   // max unknowns (2 x free nodes)
   int smem_per_warp;
-  double* scratch;  // tile tier: 12 doubles per candidate edge and CTA (12 * emax * gridDim.x), else unused
 };
 
 __host__ __device__ inline int tri(int n) { return n * (n + 1) / 2; }
@@ -666,9 +663,8 @@ __global__ void quartic_roots_kernel(const double* __restrict__ coef, const doub
   if (wid >= n) return;  // whole warps leave together
   const double q[5] = {coef[5 * wid], coef[5 * wid + 1], coef[5 * wid + 2], coef[5 * wid + 3], coef[5 * wid + 4]};
   double out[4] = {0.0, 0.0, 0.0, 0.0};
-  long long pp = 0;
-  const int c = use_grid ? quartic_roots_grid(q, lohi[2 * wid], lohi[2 * wid + 1], out, lane, pp)
-                         : quartic_roots_in(q, lohi[2 * wid], lohi[2 * wid + 1], out, lane, pp);
+  const int c = use_grid ? quartic_roots_grid(q, lohi[2 * wid], lohi[2 * wid + 1], out, lane)
+                         : quartic_roots_in(q, lohi[2 * wid], lohi[2 * wid + 1], out, lane);
   if (lane == 0) {
     counts[wid] = c;
     for (int k = 0; k < 4; ++k) roots[4 * wid + k] = out[k];

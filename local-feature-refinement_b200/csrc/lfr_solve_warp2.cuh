@@ -486,53 +486,27 @@ template <class Ctx>
 __device__ __forceinline__ void stage_edges(Ctx& C, const uint32_t* rowstart, const uint32_t* candptr, int Nc,
                                             int Eup, const DevProblem& P, int lane) {
   if (Eup == 0) return;
-  if (P.stage_mode == 1) {
-    // Pacing of zero-copy pulls: every resident warp asking for its records at once makes the PCIe
-    // link serve ~10 MB of requests round-robin, so the FIRST components (the largest, dispatched
-    // first because they run longest) get their data last.  A ticket counter keeps at most
-    // `pull_window` bytes outstanding: records arrive in dispatch order at the same link rate.
-    const bool paced = P.pull_window != 0;
-    if (paced) {
-      if (lane == 0) {
-        const unsigned long long ticket = atomicAdd(P.pull_ctr, 80ull * (unsigned)Eup);
-        const volatile unsigned long long* arrived = P.pull_ctr + 1;
-        while ((long long)(ticket - *arrived) >= (long long)P.pull_window) __nanosleep(64);
-      }
-      __syncwarp();
+  // Pacing of zero-copy pulls: every resident warp asking for its records at once makes the PCIe
+  // link serve ~10 MB of requests round-robin, so the FIRST components (the largest, dispatched
+  // first because they run longest) get their data last.  A ticket counter keeps at most
+  // `pull_window` bytes outstanding: records arrive in dispatch order at the same link rate.
+  const bool paced = P.pull_window != 0;
+  if (paced) {
+    if (lane == 0) {
+      const unsigned long long ticket = atomicAdd(P.pull_ctr, 80ull * (unsigned)Eup);
+      const volatile unsigned long long* arrived = P.pull_ctr + 1;
+      while ((long long)(ticket - *arrived) >= (long long)P.pull_window) __nanosleep(64);
     }
-    if (lane == 0) mbar_arrive_expect_tx(C.bar, 80u * (uint32_t)Eup);
     __syncwarp();
-    for (int l = lane; l < Nc; l += 32) {
-      const uint32_t d = candptr[l + 1] - candptr[l];
-      if (d) bulk_copy_g2s(C.stage + 5 * candptr[l], P.edges + 5 * (size_t)rowstart[l], 80u * d, C.bar);
-    }
-    mbar_wait(C.bar, 0);
-    if (paced && lane == 0) atomicAdd(P.pull_ctr + 1, 80ull * (unsigned)Eup);
-  } else {
-    // LDG -> STS, lane-linear over the 16-byte words, four loads in flight per lane
-    const int W = 5 * Eup;
-    for (int w0 = lane; w0 < W; w0 += 128) {
-      float4 v[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const int w = w0 + 32 * u;
-        if (w < W) {
-          const int k = w / 5, t = w - 5 * k;
-          int lo = 0, hi = Nc - 1;
-          while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if ((int)candptr[mid] <= k) lo = mid; else hi = mid - 1;
-          }
-          v[u] = __ldg(P.edges + 5 * (size_t)(rowstart[lo] + (uint32_t)(k - (int)candptr[lo])) + t);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const int w = w0 + 32 * u;
-        if (w < W) C.stage[w] = v[u];
-      }
-    }
   }
+  if (lane == 0) mbar_arrive_expect_tx(C.bar, 80u * (uint32_t)Eup);
+  __syncwarp();
+  for (int l = lane; l < Nc; l += 32) {
+    const uint32_t d = candptr[l + 1] - candptr[l];
+    if (d) bulk_copy_g2s(C.stage + 5 * candptr[l], P.edges + 5 * (size_t)rowstart[l], 80u * d, C.bar);
+  }
+  mbar_wait(C.bar, 0);
+  if (paced && lane == 0) atomicAdd(P.pull_ctr + 1, 80ull * (unsigned)Eup);
   __syncwarp();
 }
 
@@ -543,7 +517,7 @@ __device__ __forceinline__ void warp_setup(Ctx& C, uint32_t* rowstart, uint32_t*
   const uint32_t nbeg = P.comp_ptr[c];
   const int Nc = (int)(P.comp_ptr[c + 1] - nbeg);
   C.Nc = Nc;
-  if (P.stage_mode == 1 && lane == 0) mbar_init(C.bar, 1);
+  if (lane == 0) mbar_init(C.bar, 1);
   int run = 0;
   for (int l0 = 0; l0 < Nc; l0 += 32) {
     const int l = l0 + lane;

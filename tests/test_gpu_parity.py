@@ -150,49 +150,44 @@ def _compare_dbg(b200, oracle, p, debug_flags, **opts):
     return pos_g, st_g
 
 
-@pytest.mark.parametrize("flags,cfg", [("FORCE_SMEM_CHOLESKY", "cfg1"), ("FORCE_SMEM_CHOLESKY", "cfg3"),
-                                       ("NO_TILE", "cfg4"), ("TILE_FROM_1", "cfg2")])
-def test_fallback_tiers_match_oracle(b200, oracle, flags, cfg):
+@pytest.mark.parametrize("flags,cfg", [("FORCE_SMEM_CHOLESKY", "cfg1"), ("FORCE_SMEM_CHOLESKY", "cfg2"),
+                                       ("FORCE_SMEM_CHOLESKY", "cfg3"), ("NO_TILE", "cfg4")])
+def test_forced_fallback_tiers_match_oracle(b200, oracle, flags, cfg):
     """The shared-memory Cholesky warp kernel (solve_warp_kernel) is the tier for
     80 < n <= 96 unknowns and the fallback behind the register kernels; lfr_options.debug_flags
     (LFR_DBG_*) route the same scenes through it (cfg4 without the tile tier: v1 for
-    32 < n <= 96).  TILE_FROM = 1 routes every component with n <= 32 to the two-warp tile
-    kernel <64, 32> instead of the one-warp kernel."""
+    32 < n <= 96; cfg2, the flagship scene, with every warp-tier component on it)."""
     from lfr_b200 import capi
-    dbg = {"FORCE_SMEM_CHOLESKY": capi.DBG_FORCE_SMEM_CHOLESKY, "NO_TILE": capi.DBG_NO_TILE,
-           "TILE_FROM_1": 1 << capi.DBG_TILE_FROM_SHIFT}[flags]
+    dbg = {"FORCE_SMEM_CHOLESKY": capi.DBG_FORCE_SMEM_CHOLESKY, "NO_TILE": capi.DBG_NO_TILE}[flags]
     _, p = get_problem(cfg)
     _compare_dbg(b200, oracle, p, dbg)
 
 
 @pytest.mark.parametrize("cfg", ["cfg2", "cfg4", "ring60"])
-def test_staging_and_zero_copy_variants_are_bitwise_identical(b200, oracle, cfg):
+def test_zero_copy_and_hbm_solves_are_bitwise_identical(b200, oracle, cfg):
     """The same solve with (a) TMA bulk staging from the caller's pinned buffers (zero-copy: edge
     records pulled over PCIe straight into shared memory, results written straight back), (b) the
-    same through HBM, (c) LDG -> STS staging: identical bits, all equal to the oracle to 1e-4 px.
+    same through HBM: identical bits, both equal to the oracle to 1e-4 px.
     ring60 adds the CTA tier: its preparation kernel copies the kept records out of the pinned array."""
     import ctypes as C
     import torch
     from lfr_b200 import capi
     _, p = get_problem(cfg)
     pos_ref, st_ref = _compare_dbg(b200, oracle, p, capi.DBG_NO_ZERO_COPY)
-    pos_ldg, st_ldg = b200.solve(p, b200.default_options(debug_flags=capi.DBG_NO_ZERO_COPY | capi.DBG_STAGE_LDG))
-    assert np.array_equal(pos_ref, pos_ldg) and np.array_equal(st_ref["iterations"], st_ldg["iterations"])
     # pinned caller buffers -> zero-copy
     s, keep = b200.marshal(p)
     e_pin = torch.empty(keep["edges"].nbytes, dtype=torch.uint8).pin_memory()
     e_pin.numpy()[:] = keep["edges"].view(np.uint8).reshape(-1)
     s.edges = e_pin.data_ptr()
     N = p.graph.n_nodes
-    for dbg in (0, capi.DBG_STAGE_LDG):
-        pos_pin = torch.zeros(2 * N, dtype=torch.float64).pin_memory()
-        st, bufs = b200.make_stats(p.n_components)
-        o = b200.default_options(debug_flags=dbg)
-        rc = b200.lib.lfr_solve(C.byref(s), C.byref(o), C.c_void_p(pos_pin.data_ptr()), C.byref(st))
-        b200.check(rc, "lfr_solve")
-        assert np.array_equal(pos_pin.numpy().reshape(N, 2), pos_ref), dbg
-        assert np.array_equal(bufs["iterations"], st_ref["iterations"])
-        assert np.array_equal(bufs["termination"], st_ref["termination"])
+    pos_pin = torch.zeros(2 * N, dtype=torch.float64).pin_memory()
+    st, bufs = b200.make_stats(p.n_components)
+    o = b200.default_options()
+    rc = b200.lib.lfr_solve(C.byref(s), C.byref(o), C.c_void_p(pos_pin.data_ptr()), C.byref(st))
+    b200.check(rc, "lfr_solve")
+    assert np.array_equal(pos_pin.numpy().reshape(N, 2), pos_ref)
+    assert np.array_equal(bufs["iterations"], st_ref["iterations"])
+    assert np.array_equal(bufs["termination"], st_ref["termination"])
 
 
 def _quartic_cases(rng, n):

@@ -13,8 +13,8 @@ timeout 300 python tools/gpu_cycles.py cfg2 > $O/r02_cycles_cfg2.txt 2>&1
 timeout 300 python tools/gpu_zc_timeline.py cfg2 0 > $O/r02_timeline_zero_copy.txt 2>&1
 timeout 300 python tools/gpu_zc_timeline.py cfg2 8 > $O/r02_timeline_hbm.txt 2>&1
 timeout 600 python tools/gpu_batched.py > $O/r02_batched.txt 2>&1
-timeout 600 python tools/gpu_pull_window.py cfg2 0 256 512 1024 > $O/r02_pull_window_cfg2.txt 2>&1
-timeout 600 python tools/gpu_pull_window.py cfg5 512 > $O/r02_e2e_cfg5.txt 2>&1
+timeout 600 python tools/gpu_e2e_timeline.py cfg2 > $O/r02_e2e_cfg2.txt 2>&1
+timeout 600 python tools/gpu_e2e_timeline.py cfg5 > $O/r02_e2e_cfg5.txt 2>&1
 timeout 900 python tools/gpu_cfg5.py cfg5 > $O/r02_cfg5_madrid_scale_1gpu.json 2> $O/r02_cfg5.err
 timeout 900 python tools/gpu_cta_parity.py > $O/r02_cta_parity.txt 2>&1
 timeout 600 python tools/gpu_tier_timeline.py cfg4 > $O/r02_tier_timeline_cfg4.txt 2>&1
@@ -27,9 +27,8 @@ timeout 1500 ncu --set full --clock-control none --import-source on -k regex:sol
 ncu -i $O/r02_cta_full.ncu-rep --page raw --csv > $O/r02_cta_full_raw.csv 2>/dev/null
 ncu -i $O/r02_cta_full.ncu-rep --page details > $O/r02_cta_full_details.txt 2>/dev/null
 rm -f $O/r02_cta_full.ncu-rep
-python local-feature-refinement_b200/csrc/build.py --poly-prof > /dev/null 2>&1 && timeout 300 python tools/gpu_polyprof.py cfg2 > $O/r02_polyprof.txt 2>&1
 tail -n 3 $O/r02_pytest_gpu.txt; tail -n 2 $O/r02_smoke.txt
-head -12 $O/r02_cycles_cfg2.txt; cat $O/r02_pull_window_cfg2.txt $O/r02_e2e_cfg5.txt; grep -E "solve_ms|host_stage_s|plan_create_s" $O/r02_cfg5_madrid_scale_1gpu.json; tail -n 4 $O/r02_sanitizer.txt
+head -12 $O/r02_cycles_cfg2.txt; cat $O/r02_e2e_cfg2.txt $O/r02_e2e_cfg5.txt; grep -E "solve_ms|host_stage_s|plan_create_s" $O/r02_cfg5_madrid_scale_1gpu.json; tail -n 4 $O/r02_sanitizer.txt
 python - <<'PY'
 import json,glob
 for f in sorted(glob.glob('gpurun_out/r02_bench_*.json')):

@@ -1,5 +1,13 @@
-"""A/B of a library variant built with csrc/build.py::build_variant: device-resident solve time on
-cfg2 / cfg3 and 16-scene throughput.   python tools/gpu_variant.py <lib.so> [<lib2.so> ...]"""
+"""A/B of two or more builds of the product library: per library and workload, the median
+device-resident solve time (lfr_plan_solve on a plan in HBM, CUDA events, L2 overwritten before each
+solve) and a SHA-1 of the positions and iteration counts the solve returns.  Libraries take turns
+round by round, so drift of the card or of other work on the host affects them alike.
+
+    python tools/gpu_variant.py <a.so> <b.so> [...] [--workloads cfg2,cfg3,cfg4] [--rounds 15] [--per-round 3]
+
+Relative library paths are taken from the current directory."""
+import argparse
+import hashlib
 import os
 import sys
 
@@ -10,31 +18,52 @@ import torch  # noqa: E402
 
 from lfr_b200 import build_problem, synth  # noqa: E402
 from lfr_b200 import capi  # noqa: E402
-from lfr_b200.matchset import MatchSet  # noqa: E402
-
-probs = {}
-for name in ("cfg2", "cfg3"):
-    probs[name] = build_problem(synth.generate(name))
-scenes = []
 
 
-flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-for path in sys.argv[1:]:
-    lib = capi.Library(os.path.join(R, "local-feature-refinement_b200", "csrc", path) if not os.path.isabs(path) else path)
-    for name, p in probs.items():
-        plan = capi.Plan(lib, p)
-        s = torch.cuda.current_stream().cuda_stream
-        for _ in range(3):
-            plan.solve(s)
-        torch.cuda.synchronize()
-        ts = []
-        for _ in range(15):
-            flush.zero_()
-            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record()
-            plan.solve(s)
-            b.record()
-            torch.cuda.synchronize()
-            ts.append(a.elapsed_time(b))
-        print("%-28s %-10s median %.4f ms  min %.4f ms" % (os.path.basename(path), name, float(np.median(ts)), min(ts)), flush=True)
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("libs", nargs="+")
+    ap.add_argument("--workloads", default="cfg2,cfg3,cfg4")
+    ap.add_argument("--rounds", type=int, default=15)
+    ap.add_argument("--per-round", type=int, default=3)
+    args = ap.parse_args()
+    libs = [capi.Library(os.path.abspath(path)) for path in args.libs]
+    names = args.workloads.split(",")
+    s = torch.cuda.current_stream().cuda_stream
+    plans = {}
+    for name in names:
+        p = build_problem(synth.generate(name))
+        for li, lib in enumerate(libs):
+            plan = capi.Plan(lib, p)
+            for _ in range(3):
+                plan.solve(s)
+            plans[li, name] = plan
+    torch.cuda.synchronize()
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
+    times = {k: [] for k in plans}
+    for r in range(args.rounds):
+        for name in names:
+            for j in range(len(libs)):
+                li = (r + j) % len(libs)
+                for _ in range(args.per_round):
+                    flush.fill_(r & 1)
+                    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                    a.record()
+                    plans[li, name].solve(s)
+                    b.record()
+                    torch.cuda.synchronize()
+                    times[li, name].append(a.elapsed_time(b))
+    for name in names:
+        for li, path in enumerate(args.libs):
+            pos, st = plans[li, name].download(s)
+            sha = hashlib.sha1(pos.tobytes() + np.ascontiguousarray(st["iterations"]).tobytes()).hexdigest()[:16]
+            ts = np.array(times[li, name])
+            print("%-10s %-28s median %9.4f ms  min %9.4f  p10 %9.4f  p90 %9.4f  n %3d  sha1 %s" % (
+                name, os.path.basename(path), np.median(ts), ts.min(), np.percentile(ts, 10), np.percentile(ts, 90),
+                ts.size, sha), flush=True)
+    for plan in plans.values():
         plan.close()
+
+
+if __name__ == "__main__":
+    main()
